@@ -13,6 +13,10 @@ the outputs are all-gathered over NCCL.  Prints ONE JSON line (rank 0).
   cpu_baseline the reference algorithm (oracle port, torch CPU ops) on this box's host cores
   parity       max-abs / mean-abs error of image 0 of the timed batch vs the CPU reference algorithm (same run)
   clocks       SM clock / throttle reasons sampled during the timed region
+
+--dump-outputs DIR writes the images the timed path returned in its last step to DIR/img.npy (float32, NCHW; a batch
+above 64 MB is cut to a fixed seeded sample of whole images).  Inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -28,6 +32,7 @@ if ROOT not in sys.path:
 
 import torch  # noqa: E402
 
+DUMP_BYTES = 64_000_000
 HBM_FALLBACK_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 print_json = print
 
@@ -53,12 +58,30 @@ def parse_args():
                          "with 8 SMs left free for its 8 channels (nccl), or whichever measured faster at this world size (auto: ce at 2 GPUs, nccl above)")
     ap.add_argument("--masks", default="free_form", choices=["free_form", "blocks"], help="synthetic hole masks")
     ap.add_argument("--profile-out", default=None, help="write the per-launch table (JSON) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the images of the last timed step to DIR/img.npy (float32; at most 64 MB, a seeded sample of whole images)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.res is None:
         args.res = 512 if args.workload == "migan" else 256
     if args.batch is None:
         args.batch = 32 if args.workload == "migan" else 16
     return args
+
+
+def dump_outputs(out_dir: str, img: torch.Tensor) -> None:
+    """img [N, 3, R, R] -> out_dir/img.npy as float32; above DUMP_BYTES, a seeded choice of whole images (in batch order)."""
+    import numpy as np
+
+    img = img.detach().to("cpu", torch.float32)
+    keep = min(img.shape[0], (DUMP_BYTES - 128) // (img[0].numel() * 4))      # 128: the .npy header
+    if keep < img.shape[0]:
+        pick = torch.randperm(img.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        print("dump-outputs: images %s of %d" % (pick.tolist(), img.shape[0]), file=sys.stderr)
+        img = img[pick]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "img.npy"), img.contiguous().numpy())
 
 
 # ------------------------------------------------------------------------------------------
@@ -192,8 +215,10 @@ def run_reference(args):
         O.generator_forward(sd, x, args.res)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.generator_forward(sd, x, args.res)
+        y = O.generator_forward(sd, x, args.res)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     value = args.steps / dt
     line = {
         "impl": "reference", "metric": "images/sec", "value": value, "unit": "images/s",
@@ -269,6 +294,8 @@ def run_b200(args):
     barrier()
     clocks = sampler.stop()
     elapsed_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:                # h: the last step's output (its gather handle at N > 1)
+        dump_outputs(args.dump_outputs, h if sharded is None else h.wait())
     if world > 1:
         t = torch.tensor([elapsed_ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -502,6 +529,8 @@ def run_comodgan(args):
     torch.cuda.synchronize(dev)
     clocks = sampler.stop()
     elapsed_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y)
     y_host = torch.empty((B, 3, R, R), dtype=torch.float32).pin_memory()
     t0 = time.perf_counter()
     for _ in range(K):

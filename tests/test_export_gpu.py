@@ -1,6 +1,6 @@
 """Training snapshot -> inference weights on the B200 (SURVEY.md 8(f) row f3, scripts/export_inference_model.py:17-85):
 `migan_b200.export.reparam_filter` / `copy_weights` against oracle/export_oracle.py (pinned to the reference's own
-`get_source_w` by tests/test_host.py where the reference exists).  The source here is a module tree with the training
+`get_source_w` by tests/test_host.py through tests/golden/scripts.npz).  The source here is a module tree with the training
 generator's attribute layout (lib/model_zoo/migan.py) built from plain containers -- the reference is absent on the GPU box.
 Bar: relative error < 1e-6 per filter (fp64 sum of squares vs torch's fp32 tree), and the exported generator's forward
 equals the oracle's forward on the oracle-exported weights within the generator's own tolerance."""

@@ -2,6 +2,7 @@
 import ctypes
 import os
 import re
+import subprocess
 import sys
 
 import pytest
@@ -77,11 +78,15 @@ def test_constructor_and_cpu_errors(lib):
 
 
 def test_no_cuda_device_fails_loudly(lib):
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    h = ctypes.c_void_p()
-    assert lib.migan_create(64, 0, ctypes.byref(h)) == _abi.ERR_CUDA
-    assert b"no CPU path" in lib.migan_last_error()
+    """Run in a child process with no CUDA device visible (CUDA_VISIBLE_DEVICES empty), so that it holds on a GPU machine too."""
+    code = ("import ctypes, sys; sys.path.insert(0, %r); from migan_b200 import _abi; lib = _abi.load(); h = ctypes.c_void_p(); "
+            "print(lib.migan_create(64, 0, ctypes.byref(h))); print(lib.migan_last_error().decode())" % ROOT)
+    child = subprocess.run([sys.executable] + (["-s"] if sys.flags.no_user_site else []) + ["-c", code],
+                           env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=300)
+    assert child.returncode == 0, child.stderr[-2000:]
+    rc, msg = child.stdout.strip().split("\n", 1)
+    assert int(rc) == _abi.ERR_CUDA
+    assert "no CPU path" in msg
 
 
 def test_product_does_not_import_oracle():
@@ -150,65 +155,98 @@ def test_comodgan_constructor_and_cpu_errors(lib):
     lib.comodgan_destroy(h)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib/model_zoo"), reason="reference checkout not present (GPU box)")
-def test_dropin_rebinds_reference_modules(lib, monkeypatch):
+def _scripts_golden():
+    """What the reference's scripts did with these classes (tests/golden/make_golden_scripts.py)."""
+    import numpy as np
+    return np.load(os.path.join(ROOT, "tests", "golden", "scripts.npz"))
+
+
+def test_dropin_rebinds_reference_modules(lib, monkeypatch, tmp_path):
     """python -m migan_b200.dropin scripts.demo ...: the reference's import sites (scripts/demo.py:15-21) resolve to the
-    B200 classes without editing any reference file.  Build container only."""
+    B200 classes without editing any reference file.  Stand-in modules take the place of the reference's
+    lib.model_zoo.migan_inference / lib.model_zoo.comodgan; the Co-Mod-GAN built through the rebound names has the
+    state_dict keys of the reference's own construction (scripts/demo.py:95-100, stored)."""
     import importlib
-    import warnings
-    monkeypatch.syspath_prepend("/root/reference")
-    warnings.filterwarnings("ignore")
+    (tmp_path / "lib" / "model_zoo").mkdir(parents=True)
+    (tmp_path / "lib" / "__init__.py").write_text("")
+    (tmp_path / "lib" / "model_zoo" / "__init__.py").write_text("")
+    (tmp_path / "lib" / "model_zoo" / "migan_inference.py").write_text("class Generator:\n    pass\n")
+    (tmp_path / "lib" / "model_zoo" / "comodgan.py").write_text("".join("class %s:\n    pass\n" % n for n in ("Generator", "Mapping", "Encoder", "Synthesis")))
+    monkeypatch.syspath_prepend(str(tmp_path))
     from migan_b200 import comodgan, dropin
-    ref_mi = importlib.import_module("lib.model_zoo.migan_inference")
-    ref_cm = importlib.import_module("lib.model_zoo.comodgan")
-    saved = (ref_mi.Generator, ref_cm.Generator, ref_cm.Mapping, ref_cm.Encoder, ref_cm.Synthesis)
     try:
+        ref_mi = importlib.import_module("lib.model_zoo.migan_inference")
+        ref_cm = importlib.import_module("lib.model_zoo.comodgan")
+        saved = (ref_mi.Generator, ref_cm.Generator)
         dropin.install()
         assert ref_mi.Generator is migan_b200.Generator and ref_mi.ReferenceGenerator is saved[0]
         assert ref_cm.Generator is comodgan.Generator and ref_cm.ReferenceGenerator is saved[1]
-        # the construction of scripts/demo.py:95-100, through the patched names
+        assert (ref_cm.Mapping, ref_cm.Encoder, ref_cm.Synthesis) == (comodgan.Mapping, comodgan.Encoder, comodgan.Synthesis)
         model = ref_cm.Generator(ref_cm.Mapping(num_ws=14), ref_cm.Encoder(resolution=256), ref_cm.Synthesis(resolution=256))
-        ref_keys = list(saved[1](saved[2](num_ws=14), saved[3](resolution=256), saved[4](resolution=256)).state_dict().keys())
-        assert list(model.state_dict().keys()) == ref_keys
+        assert list(model.state_dict().keys()) == [str(k) for k in _scripts_golden()["comodgan256_keys"]]
     finally:
-        ref_mi.Generator, ref_cm.Generator, ref_cm.Mapping, ref_cm.Encoder, ref_cm.Synthesis = saved
+        for name in ("lib.model_zoo.comodgan", "lib.model_zoo.migan_inference", "lib.model_zoo", "lib"):
+            sys.modules.pop(name, None)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib/model_zoo"), reason="reference checkout not present (GPU box)")
-def test_reference_export_script_accepts_b200_generator(lib, monkeypatch):
+def _export_source(z):
+    """The training generator's tensors that the reference's `copy_weights` read, regenerated from the stored names,
+    shapes and seed (training parameters as nn.Parameter, noise planes as plain buffers)."""
+    from oracle import export_oracle as E
+    names = [str(n) for n in z["src_names"]]
+    shapes = [tuple(int(d) for d in s[:n]) for s, n in zip(z["src_shapes"], z["src_ndim"])]
+    src = E.seeded_source(names, shapes, int(z["src_seed"]))
+    return {k: (torch.nn.Parameter(v) if p else v) for (k, v), p in zip(src.items(), z["src_is_param"])}
+
+
+def _source_filters(src, conv):
+    """[w0 .. w{k-1}] of a re-parameterised training conv, [weight] of a plain one."""
+    ws = [src["%s.w%d" % (conv, i)] for i in range(16) if "%s.w%d" % (conv, i) in src]
+    return [w.detach() for w in (ws or [src[conv + ".weight"]])]
+
+
+def _sample(t, z, key):
+    return t.detach().reshape(-1)[torch.from_numpy(z["idx." + key]).long()]
+
+
+def test_reference_export_script_accepts_b200_generator(lib):
     """scripts/export_inference_model.py:17-85 `copy_weights(source_G, dest)` -- the reference's route from a training
     snapshot (re-parameterised train graph, lib/model_zoo/migan.py) to inference weights -- works with the B200 class as
-    `dest` (attribute paths, `fromrgb is None`, `conv2.bias is None`, `use_noise`), and gives the same state_dict as with
-    the reference's own inference Generator.  Also the reference's behavioural pin: train graph == inference graph
-    (export_inference_model.py:149-151), here against the oracle.  Build container only."""
-    import importlib
-    import warnings
-    monkeypatch.syspath_prepend("/root/reference")
-    warnings.filterwarnings("ignore")
-    M = importlib.import_module("lib.model_zoo.migan")
-    ref_inf = importlib.import_module("lib.model_zoo.migan_inference")
-    exp = importlib.import_module("scripts.export_inference_model")
-    R = 64
-    torch.manual_seed(0)
-    src = M.Generator(M.Encoder(resolution=R, ic_n=4, depthwise=True, reparametrize=True, num_reparam_tensors=9),
-                      M.Synthesis(resolution=R, depthwise=True, reparametrize=True, num_reparam_tensors=9)).eval()
-    with torch.no_grad():
-        for name, p in src.named_parameters():
-            if name.endswith("bias"):
-                p.copy_(0.2 * torch.randn_like(p))
-            if name.endswith("noise_strength"):
-                p.fill_(0.3)
-    ref, mine = ref_inf.Generator(resolution=R).eval(), migan_b200.Generator(R).eval()
-    exp.copy_weights(src, ref, resolution=R)
-    exp.copy_weights(src, mine, resolution=R)
-    a, b = ref.state_dict(), mine.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    assert all(torch.equal(a[k], b[k]) for k in a)
+    `dest`.  The script's run on its own inference Generator is replayed on the B200 Generator from the stored trace:
+    every attribute it reads there (`fromrgb is None`, `conv2.bias is None`, `use_noise`, the blocks) must give the
+    answer the reference's class gave, and every assignment it made (filters, biases, noise tensors, blocks) is made
+    again, with the same source.  The B200 Generator's state_dict then equals what the reference exported (stored
+    sample).  Also the reference's behavioural pin: train graph == inference graph (export_inference_model.py:149-151),
+    here the stored training-graph output against the oracle."""
+    import torch.nn as nn
+    from oracle import export_oracle as E
+    z = _scripts_golden()
+    src, R = _export_source(z), int(z["resolution"])
+    mine = migan_b200.Generator(R).eval()
+    keys = [str(k) for k in z["dest_keys"]]
+    assert list(mine.state_dict().keys()) == keys
+    for op, path, info in zip(z["trace_op"], z["trace_path"], z["trace_info"]):
+        parent, _, leaf = str(path).rpartition(".")
+        node = mine.get_submodule(parent)
+        if op == "get":
+            assert E.attribute_kind(getattr(node, leaf)) == info, path
+            continue
+        if info == "block":                                   # setattr(dest.encoder, f"b{res}", dest_module)
+            value = getattr(node, leaf)
+        else:
+            kind, how, from_path = str(info).split(":")
+            value = E.merged_filter(_source_filters(src, from_path)) if how == "filter" else src[from_path]
+            if kind == "Parameter" and not isinstance(value, nn.Parameter):
+                value = nn.Parameter(value)
+        setattr(node, leaf, value)
+    b = mine.state_dict()
+    assert list(b.keys()) == keys
+    for key in keys:
+        assert torch.equal(_sample(b[key], z, key), torch.from_numpy(z["val." + key])), key
     x = O.make_input(R, 2)
-    with torch.no_grad():
-        y_src = src(x, noise_mode="const")
     y_or = O.generator_forward({k: v.detach() for k, v in b.items()}, x, R)
-    assert float((y_src - y_or).abs().max()) < 1e-4            # SURVEY 8c pin (1): 1.05e-5 at output scale 13.6
+    y_src = torch.from_numpy(z["y_val"])
+    assert float((y_or.reshape(-1)[torch.from_numpy(z["y_idx"]).long()] - y_src).abs().max()) < 1e-4   # SURVEY 8c pin (1)
 
 
 def test_resolutions_above_512_are_rejected_up_front(lib):
@@ -250,39 +288,21 @@ def test_export_kernel_matches_oracle_in_emulation():
         assert torch.allclose(got.flatten(1).square().sum(1), torch.ones(shape[0]), atol=1e-5)   # unit L2 filters
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib/model_zoo"), reason="reference checkout not present (GPU box)")
-def test_export_matches_reference_copy_weights(monkeypatch):
+def test_export_matches_reference_copy_weights():
     """oracle/export_oracle.merged_filter == the reference's `get_source_w` (through its effect: `copy_weights` into the
-    reference's inference Generator), and the export kernel (emulation) reproduces every filter of that state_dict.
-    Build container only."""
-    import importlib
-    import warnings
+    reference's inference Generator, stored sample), and the export kernel (emulation) reproduces every filter of that
+    state_dict."""
     from oracle import export_oracle as E
-    monkeypatch.syspath_prepend("/root/reference")
-    warnings.filterwarnings("ignore")
-    M = importlib.import_module("lib.model_zoo.migan")
-    ref_inf = importlib.import_module("lib.model_zoo.migan_inference")
-    exp = importlib.import_module("scripts.export_inference_model")
-    R = 64
-    torch.manual_seed(1)
-    src = M.Generator(M.Encoder(resolution=R, ic_n=4, depthwise=True, reparametrize=True, num_reparam_tensors=9),
-                      M.Synthesis(resolution=R, depthwise=True, reparametrize=True, num_reparam_tensors=9)).eval()
-    ref = ref_inf.Generator(resolution=R).eval()
-    exp.copy_weights(src, ref, resolution=R)
-    sd = ref.state_dict()
+    z = _scripts_golden()
+    src = _export_source(z)
     checked = 0
-    for side in ("encoder", "synthesis"):
-        for res in (4, 8, 16, 32, 64):
-            blk = getattr(getattr(src, side), "b%d" % res)
-            convs = [("conv1.conv1", blk.conv1.conv1), ("conv1.conv2", blk.conv1.conv2), ("conv2.conv1", blk.conv2.conv1), ("conv2.conv2", blk.conv2.conv2)]
-            head = "fromrgb" if side == "encoder" else "torgb"
-            if "%s.b%d.%s.weight" % (side, res, head) in sd:
-                convs.append((head, getattr(blk, head)))
-            for name, conv in convs:
-                ws = [getattr(conv, "w%d" % i).detach() for i in range(conv.num_reparam_tensors)] if conv.reparametrize else [conv.weight.detach()]
-                want = sd["%s.b%d.%s.weight" % (side, res, name)]
-                assert torch.equal(E.merged_filter(ws), want), (side, res, name)           # the oracle IS the reference expression
-                got = _emul_reparam(ws)
-                assert float(((got - want).abs().amax(dim=(1, 2, 3)) / want.abs().amax(dim=(1, 2, 3))).max()) < 1e-6
-                checked += 1
+    for key, info in zip(z["trace_path"], z["trace_info"]):     # the filters copy_weights wrote, with their training convs
+        if not str(info).startswith("Parameter:filter:"):
+            continue
+        key, ws = str(key), _source_filters(src, str(info).rsplit(":", 1)[1])
+        want = E.merged_filter(ws)
+        assert torch.equal(_sample(want, z, key), torch.from_numpy(z["val." + key])), key   # the oracle IS the reference expression
+        got = _emul_reparam(ws)
+        assert float(((got - want).abs().amax(dim=(1, 2, 3)) / want.abs().amax(dim=(1, 2, 3))).max()) < 1e-6
+        checked += 1
     assert checked == 46      # 5 levels x 2 sides x 4 convolutions + 1 fromrgb + 5 torgb
