@@ -141,6 +141,36 @@ int b200_pipeline_preprocess(const uint8_t* image_chw, const uint8_t* mask_hw, i
 int b200_pipeline_postprocess(const float* y_nchw, uint8_t* image_chw, const uint8_t* mask_hw, int H, int W, const int* box4_host,
                               int resolution, const float* k25_host, void* scratch, size_t scratch_bytes, void* stream);
 
+/* Batched crop pipeline: n requests of any sizes in one call, crop windows found on the device.  Request i is image_chw u8
+ * [3,H,W] (updated in place) and mask_hw u8 [mask_h,mask_w] (255 = known), DEVICE pointers; the table itself is a HOST
+ * array of at most MIGAN_PIPE_BATCH_MAX entries, passed to the kernels by value (no staging copy, no host wait).  H, W >= 3.
+ * Every stage is a fixed number of launches for the whole batch, sized on the host for crops as large as their images; the
+ * kernels read the actual windows from boxes (DEVICE int32 [n][4] = {x_min, x_max, y_min, y_max}), which the host never reads:
+ *   b200_pipeline_batch_boxes       masks at another size -> image size (nearest); hole extents of every mask in one pass
+ *                                   (16-byte loads, warp reductions, atomics); extents -> crop windows (the arithmetic of
+ *                                   migan_crop_box) -> boxes.  3 launches, 4 when some mask needs resizing.
+ *   b200_pipeline_batch_preprocess  weight tables, width pass, height pass fused with round + normalisation -> row i of
+ *                                   x[n,4,res,res].  3 launches.
+ *   [generator forward at batch n: y[n,3,res,res]]
+ *   b200_pipeline_batch_postprocess weight tables, width pass of y, height pass fused into the feathered blend -> image[crop].
+ *                                   3 launches.
+ * Results equal b200_pipeline_preprocess / _postprocess per request bit for bit.  scratch: b200_pipeline_batch_scratch_bytes
+ * bytes of device memory (16-byte aligned), the same area for the three calls of a batch (the resized masks live there). */
+#define MIGAN_PIPE_BATCH_MAX 64
+typedef struct migan_pipe_req {
+    uint8_t* image_chw;
+    const uint8_t* mask_hw;
+    int H, W;
+    int mask_h, mask_w;
+} migan_pipe_req;
+size_t b200_pipeline_batch_scratch_bytes(const migan_pipe_req* reqs_host, int n, int resolution);
+int b200_pipeline_batch_boxes(const migan_pipe_req* reqs_host, int n, int resolution, int padding, int* boxes_dev,
+                              void* scratch, size_t scratch_bytes, void* stream);
+int b200_pipeline_batch_preprocess(const migan_pipe_req* reqs_host, int n, int resolution, const int* boxes_dev, float* x_nchw,
+                                   void* scratch, size_t scratch_bytes, void* stream);
+int b200_pipeline_batch_postprocess(const float* y_nchw, const migan_pipe_req* reqs_host, int n, int resolution, const int* boxes_dev,
+                                    const float* k25_host, void* scratch, size_t scratch_bytes, void* stream);
+
 /* Training snapshot -> inference filter, scripts/export_inference_model.py:18-27 (`get_source_w`): out[cout][fan] =
  * v * rsqrt(sum_fan v^2 + 1e-8) with v = (w_0 + ... + w_{k-1}) / sqrt(k) for a re-parameterised layer (k tensors) or v = w_0
  * (k = 1).  w_dev: HOST array of k DEVICE pointers to [cout][fan] fp32 tensors (fan = cin/groups * kh * kw); out: device.

@@ -42,6 +42,10 @@ SYMBOLS = [
     ("migan_crop_box", c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     ("b200_pipeline_preprocess", c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     ("b200_pipeline_postprocess", c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    ("b200_pipeline_batch_scratch_bytes", c_size_t, [c_void_p, c_int, c_int]),
+    ("b200_pipeline_batch_boxes", c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    ("b200_pipeline_batch_preprocess", c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    ("b200_pipeline_batch_postprocess", c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     ("b200_reparam_filter", c_int, [c_void_p, c_int, c_int, c_int64, c_void_p, c_void_p]),
     ("b200_stream_memops_available", c_int, []),
     ("b200_stream_wait_value32", c_int, [c_void_p, c_void_p, ctypes.c_uint32]),
@@ -80,7 +84,15 @@ COMOD_SYMBOLS = [
      [c_void_p, c_size_t, POINTER(c_size_t), POINTER(c_int), POINTER(c_int), c_void_p]),
 ]
 
-PREPOST_SYMBOLS = [s for s in SYMBOLS if s[0] in ("b200_preprocess_u8", "b200_postprocess_u8", "b200_feather_composite")]
+PIPE_BATCH_MAX = 64   # MIGAN_PIPE_BATCH_MAX
+
+
+class PipeReq(ctypes.Structure):
+    """migan_pipe_req: one request of a batched crop-pipeline call (device pointers, sizes)."""
+    _fields_ = [("image_chw", c_void_p), ("mask_hw", c_void_p), ("H", c_int), ("W", c_int), ("mask_h", c_int), ("mask_w", c_int)]
+
+
+PREPOST_SYMBOLS =[s for s in SYMBOLS if s[0] in ("b200_preprocess_u8", "b200_postprocess_u8", "b200_feather_composite")]
 
 _lib = None
 

@@ -6,6 +6,8 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 
+#include "../../include/migan_b200.h"
+
 namespace migan {
 
 // Per-device one-time setup (dynamic shared memory opt-in); called by migan_create.
@@ -81,6 +83,12 @@ int launch_pipeline_preprocess(const uint8_t* image, const uint8_t* mask, int H,
                                void* scratch, cudaStream_t s);
 int launch_pipeline_postprocess(const float* y, uint8_t* image, const uint8_t* mask, int H, int W, const int* box, int res,
                                 const float* k25_host, void* scratch, cudaStream_t s);
+// batched form (migan_pipe_req of include/migan_b200.h; boxes on the device)
+size_t pipeline_batch_scratch_bytes(const migan_pipe_req* reqs, int n, int res);
+int launch_pipeline_batch_boxes(const migan_pipe_req* reqs, int n, int res, int padding, int* boxes, void* scratch, cudaStream_t s);
+int launch_pipeline_batch_preprocess(const migan_pipe_req* reqs, int n, int res, const int* boxes, float* x, void* scratch, cudaStream_t s);
+int launch_pipeline_batch_postprocess(const float* y, const migan_pipe_req* reqs, int n, int res, const int* boxes,
+                                      const float* k25_host, void* scratch, cudaStream_t s);
 
 
 // ---- training snapshot -> inference filters (reparam.cu): scripts/export_inference_model.py:18-27 ------

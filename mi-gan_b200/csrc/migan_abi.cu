@@ -1340,6 +1340,52 @@ int b200_pipeline_postprocess(const float* y, uint8_t* image, const uint8_t* mas
     return MIGAN_OK;
 }
 
+static int check_batch(const char* who, const migan_pipe_req* reqs, int n, int res, const void* scratch, size_t scratch_bytes) {
+    if (!reqs || !scratch) return fail(MIGAN_ERR_INVALID, "%s: null argument", who);
+    if (n < 1 || n > MIGAN_PIPE_BATCH_MAX) return fail(MIGAN_ERR_INVALID, "%s: %d requests (1 to %d per call)", who, n, MIGAN_PIPE_BATCH_MAX);
+    if (res < 3) return fail(MIGAN_ERR_INVALID, "%s: bad resolution %d", who, res);
+    for (int i = 0; i < n; ++i) {
+        const migan_pipe_req& q = reqs[i];
+        if (!q.image_chw || !q.mask_hw) return fail(MIGAN_ERR_INVALID, "%s: request %d: null image or mask", who, i);
+        if (q.H < 3 || q.W < 3 || q.mask_h < 1 || q.mask_w < 1 || (int64_t)q.H * q.W >= ((int64_t)1 << 31))
+            return fail(MIGAN_ERR_INVALID, "%s: request %d: image %d x %d (at least 3 x 3, under 2^31 pixels), mask %d x %d", who, i,
+                        q.H, q.W, q.mask_h, q.mask_w);
+    }
+    if (reinterpret_cast<uintptr_t>(scratch) % 16) return fail(MIGAN_ERR_WORKSPACE, "%s: scratch is not 16-byte aligned", who);
+    const size_t need = migan::pipeline_batch_scratch_bytes(reqs, n, res);
+    if (scratch_bytes < need) return fail(MIGAN_ERR_WORKSPACE, "%s: scratch of %zu bytes, need %zu", who, scratch_bytes, need);
+    return MIGAN_OK;
+}
+
+size_t b200_pipeline_batch_scratch_bytes(const migan_pipe_req* reqs, int n, int res) {
+    if (!reqs || n < 1 || n > MIGAN_PIPE_BATCH_MAX || res < 1) return 0;
+    return migan::pipeline_batch_scratch_bytes(reqs, n, res);
+}
+
+int b200_pipeline_batch_boxes(const migan_pipe_req* reqs, int n, int res, int padding, int* boxes, void* scratch, size_t scratch_bytes,
+                              void* stream) {
+    if (int rc = check_batch("pipeline_batch_boxes", reqs, n, res, scratch, scratch_bytes)) return rc;
+    if (!boxes || padding < 0) return fail(MIGAN_ERR_INVALID, "pipeline_batch_boxes: null boxes or padding %d < 0", padding);
+    CUDA_TRY((cudaError_t)migan::launch_pipeline_batch_boxes(reqs, n, res, padding, boxes, scratch, static_cast<cudaStream_t>(stream)));
+    return MIGAN_OK;
+}
+
+int b200_pipeline_batch_preprocess(const migan_pipe_req* reqs, int n, int res, const int* boxes, float* x, void* scratch,
+                                   size_t scratch_bytes, void* stream) {
+    if (int rc = check_batch("pipeline_batch_preprocess", reqs, n, res, scratch, scratch_bytes)) return rc;
+    if (!boxes || !x) return fail(MIGAN_ERR_INVALID, "pipeline_batch_preprocess: null argument");
+    CUDA_TRY((cudaError_t)migan::launch_pipeline_batch_preprocess(reqs, n, res, boxes, x, scratch, static_cast<cudaStream_t>(stream)));
+    return MIGAN_OK;
+}
+
+int b200_pipeline_batch_postprocess(const float* y, const migan_pipe_req* reqs, int n, int res, const int* boxes, const float* k25,
+                                    void* scratch, size_t scratch_bytes, void* stream) {
+    if (int rc = check_batch("pipeline_batch_postprocess", reqs, n, res, scratch, scratch_bytes)) return rc;
+    if (!y || !boxes || !k25) return fail(MIGAN_ERR_INVALID, "pipeline_batch_postprocess: null argument");
+    CUDA_TRY((cudaError_t)migan::launch_pipeline_batch_postprocess(y, reqs, n, res, boxes, k25, scratch, static_cast<cudaStream_t>(stream)));
+    return MIGAN_OK;
+}
+
 int migan_host_wait(migan_ctx* ctx) {
     if (!ctx) return fail(MIGAN_ERR_INVALID, "null ctx");
     if (!ctx->s_out) return MIGAN_OK;
