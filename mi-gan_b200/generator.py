@@ -24,7 +24,35 @@ import torch.nn as nn
 from . import _abi, arch
 
 
-class _Node(nn.Module):
+# Bumped whenever a parameter, buffer or sub-module of any generator tree is assigned, registered or deleted: the tensor
+# list a Generator collected for its per-call weight check is stale after that (Generator._state_version).
+_tree_edits = [0]
+
+
+class _Tracked(nn.Module):
+    def __setattr__(self, name, value):
+        if value is None or isinstance(value, (torch.Tensor, nn.Module)):
+            _tree_edits[0] += 1
+        super().__setattr__(name, value)
+
+    def __delattr__(self, name):
+        _tree_edits[0] += 1
+        super().__delattr__(name)
+
+    def register_parameter(self, name, param):
+        _tree_edits[0] += 1
+        super().register_parameter(name, param)
+
+    def register_buffer(self, name, tensor, persistent=True):
+        _tree_edits[0] += 1
+        super().register_buffer(name, tensor, persistent)
+
+    def add_module(self, name, module):
+        _tree_edits[0] += 1
+        super().add_module(name, module)
+
+
+class _Node(_Tracked):
     """Parameter container: one level of the reference's attribute tree."""
 
     def forward(self, *a, **k):  # pragma: no cover
@@ -113,8 +141,14 @@ class _Engine:
         return ws
 
 
-class Generator(nn.Module):
-    """MI-GAN inference generator, B200-native.  See module docstring."""
+class Generator(_Tracked):
+    """MI-GAN inference generator, B200-native.  See module docstring.
+
+    The weights are uploaded to the device on the first forward and again whenever they change: after `load_state_dict`,
+    `.to()`, an assignment of a parameter, buffer or sub-module anywhere in the tree (`export.copy_weights` does this),
+    `p.data = t`, and in-place edits of a parameter or buffer (`p.mul_(2)` under `torch.no_grad()`, `p.copy_(t)`).
+    In-place writes through `.data` (`p.data.mul_(2)`, `p.data[0] = 1`) bypass the tensors' version counters and go unseen:
+    follow them with `load_state_dict(self.state_dict())`."""
 
     def __init__(self, resolution: int = 256, path: Optional[str] = None):
         super().__init__()
@@ -159,14 +193,19 @@ class Generator(nn.Module):
         return _abi.PATHS[name]
 
     def _state_version(self):
-        # Cheap per-call check that the uploaded weights are still current: the tensor list is collected once (and again
-        # after load_state_dict / .to() / .cuda(), which may replace tensors) and each call only sums version counters.
-        tensors = self.__dict__.get("_state_tensors")
-        if tensors is None:
-            tensors = tuple(self.state_dict(keep_vars=True).values())
-            self.__dict__["_state_tensors"] = tensors
-            self.__dict__["_state_ptrs"] = tuple(t.data_ptr() for t in tensors)
-        return (sum(t._version for t in tensors), self.__dict__["_state_ptrs"])
+        # Cheap per-call check that the uploaded weights are still current.  The tensor list is collected again only after
+        # load_state_dict / .to() / .cuda() or an edit of some generator tree (_tree_edits); the epoch counts the times it
+        # came out different.  The cache holds the listed tensors, so `is` compares them exactly.  Each call sums version
+        # counters (in-place edits) and reads data pointers (`p.data = t` changes neither the tree nor the version).
+        d = self.__dict__
+        tensors = d.get("_state_tensors")
+        if tensors is None or d.get("_state_edits") != _tree_edits[0]:
+            edits = _tree_edits[0]
+            fresh = tuple(self.state_dict(keep_vars=True).values())
+            if tensors is None or len(fresh) != len(tensors) or any(a is not b for a, b in zip(fresh, tensors)):
+                d["_state_epoch"] = d.get("_state_epoch", 0) + 1
+            d["_state_tensors"], d["_state_edits"], tensors = fresh, edits, fresh
+        return (d["_state_epoch"], sum(t._version for t in tensors), tuple(t.data_ptr() for t in tensors))
 
     def _apply(self, fn, *args, **kwargs):
         self.__dict__["_state_tensors"] = None
@@ -338,10 +377,11 @@ class Generator(nn.Module):
 
     @torch.no_grad()
     def forward_with_tap(self, x: torch.Tensor, tap: str, shape) -> (torch.Tensor, torch.Tensor):
-        """Run forward and also return the named intermediate as NCHW (debug / parity tests)."""
+        """Run forward and also return the named intermediate as NCHW (debug / parity tests).  The intermediate is NaN
+        where the forward did not write it (a name the plan does not produce)."""
         x = self._validate(x)
         eng = self._engine(x.device)
-        buf = torch.zeros((x.shape[0],) + tuple(shape), dtype=torch.float32, device=x.device)
+        buf = torch.full((x.shape[0],) + tuple(shape), float("nan"), dtype=torch.float32, device=x.device)
         _abi.check(eng.lib.migan_set_tap(eng.handle, tap.encode(), buf.data_ptr()))
         try:
             y = self.forward(x)

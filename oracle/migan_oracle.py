@@ -214,29 +214,38 @@ def upsample2d(x: torch.Tensor, taps: torch.Tensor, filter_const: torch.Tensor) 
     return F.conv2d(x, taps, groups=x.shape[1])
 
 
+def _tap(taps, name: str, x: torch.Tensor, record: bool = True) -> torch.Tensor:
+    """Named intermediate of the forward.  ``taps`` is None, a dict that collects the intermediates (names ``record=False``
+    leave out), or an object whose ``visit(name, x)`` returns the tensor the forward continues from
+    (``oracle/unit_parity.py`` continues from tensors a kernel produced)."""
+    if taps is None:
+        return x
+    visit = getattr(taps, "visit", None)
+    if visit is not None:
+        return visit(name, x)
+    if record:
+        taps[name] = x
+    return x
+
+
 def separable_conv2d(sd: Dict[str, torch.Tensor], p: str, x: torch.Tensor,
                      taps: Optional[dict] = None) -> torch.Tensor:
     """SeparableConv2d.forward -- migan_inference.py:154-170.  Which optional stages
     run is decided by which keys exist under prefix ``p``."""
     x = F.conv2d(x, sd[p + "conv1.weight"], sd[p + "conv1.bias"], padding=1, groups=x.shape[1])
     x = lrelu_agc(x)
-    if taps is not None:
-        taps[p + "dw_act"] = x
+    x = _tap(taps, p + "dw_act", x)
     if (p + "downsample.filter.weight") in sd:
         x = downsample2d(x, sd[p + "downsample.filter.weight"])
-        if taps is not None:
-            taps[p + "down"] = x
+        x = _tap(taps, p + "down", x)
     x = F.conv2d(x, sd[p + "conv2.weight"])
-    if taps is not None:
-        taps[p + "pw"] = x
+    x = _tap(taps, p + "pw", x)
     if (p + "upsample.filter.weight") in sd:
         x = upsample2d(x, sd[p + "upsample.filter.weight"], sd[p + "upsample.filter_const"])
     if (p + "noise_const") in sd:
         x = x + sd[p + "noise_const"] * sd[p + "noise_strength"]
     x = lrelu_agc(x)
-    if taps is not None:
-        taps[p + "out"] = x
-    return x
+    return _tap(taps, p + "out", x)
 
 
 def encoder_forward(sd, x_in: torch.Tensor, resolution: int, taps=None):
@@ -250,8 +259,7 @@ def encoder_forward(sd, x_in: torch.Tensor, resolution: int, taps=None):
             y = F.conv2d(x_in, sd[p + "fromrgb.weight"], sd[p + "fromrgb.bias"])
             y = lrelu_agc(y)
             x = y if x is None else x + y
-            if taps is not None:
-                taps[p + "fromrgb"] = x
+            x = _tap(taps, p + "fromrgb", x)
         feat = separable_conv2d(sd, p + "conv1.", x, taps)
         x = separable_conv2d(sd, p + "conv2.", feat, taps)
         feats[res] = feat
@@ -265,20 +273,19 @@ def synthesis_forward(sd, x: torch.Tensor, feats, resolution: int, taps=None) ->
     """Synthesis.forward -- migan_inference.py:347-352; blocks :270-279 and :303-315."""
     p = "synthesis.b4."
     x = separable_conv2d(sd, p + "conv1.", x, taps)
-    x = x + feats[4]
+    x = _tap(taps, p + "conv1.out_skip", x + feats[4], record=False)
     x = separable_conv2d(sd, p + "conv2.", x, taps)
     img = F.conv2d(x, sd[p + "torgb.weight"], sd[p + "torgb.bias"])
-    if taps is not None:
-        taps[p + "img"] = img
+    img = _tap(taps, p + "img", img)
     for res in block_res(resolution)[1:]:
         p = "synthesis.b%d." % res
         x = separable_conv2d(sd, p + "conv1.", x, taps)
         x = x + feats[res]            # skip is added AFTER the activation (:304-305)
+        x = _tap(taps, p + "conv1.out_skip", x, record=False)
         x = separable_conv2d(sd, p + "conv2.", x, taps)
         img = upsample2d(img, sd[p + "upsample.filter.weight"], sd[p + "upsample.filter_const"])
         img = img + F.conv2d(x, sd[p + "torgb.weight"], sd[p + "torgb.bias"])
-        if taps is not None:
-            taps[p + "img"] = img
+        img = _tap(taps, p + "img", img)
     return img
 
 
@@ -292,9 +299,8 @@ def generator_forward(sd: Dict[str, torch.Tensor], x: torch.Tensor, resolution: 
         sd = {k: v.to(dtype) for k, v in sd.items()}
         x = x.to(dtype)
     x4, feats = encoder_forward(sd, x, resolution, taps)
-    if taps is not None:
-        for r, f in feats.items():
-            taps["feat%d" % r] = f
+    for r, f in feats.items():
+        _tap(taps, "feat%d" % r, f)
     return synthesis_forward(sd, x4, feats, resolution, taps)
 
 

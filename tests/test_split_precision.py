@@ -10,24 +10,10 @@ The 1x1 convs run on fp16 tensor cores as  Ah*Bh + Al*Bh + Ah*Bl  with fp32 accu
   * the chosen scales (activations * 64, weights * 2^k with max|w*2^k| in [8192, 16384)) stay inside fp16 range.
 """
 import numpy as np
+import pytest
 
-
-def split_trunc(s):
-    """Prologue split (sepconv_tc.cu split_pack2): hi = s with the low 13 mantissa bits cleared, lo = fp16(s - hi)."""
-    s = s.astype(np.float32)
-    hi32 = (s.view(np.uint32) & np.uint32(0xFFFFE000)).view(np.float32)
-    hi = hi32.astype(np.float16)
-    assert np.array_equal(hi.astype(np.float32), hi32)          # exactly representable
-    lo = (s - hi32).astype(np.float16)
-    return hi, lo
-
-
-def split_round(s):
-    """Host-side weight split (migan_abi.cu pack_sepconv): hi = fp16(s), lo = fp16(s - hi)."""
-    s = s.astype(np.float32)
-    hi = s.astype(np.float16)
-    lo = (s - hi.astype(np.float32)).astype(np.float16)
-    return hi, lo
+from oracle import unit_parity as U
+from oracle.split_model import error_ratios, split_round, split_trunc
 
 
 def dot32(a16, b16):
@@ -46,6 +32,7 @@ def test_three_pass_split_is_fp32_faithful():
     a_s, w_s = a * np.float32(64.0), w * np.float32(2.0 ** k2)
     assert np.abs(a_s).max() <= 16384 and 8192 <= np.abs(w_s).max() < 16384
     ah, al = split_trunc(a_s)
+    assert np.array_equal(ah.astype(np.float32), (a_s.view(np.uint32) & np.uint32(0xFFFFE000)).view(np.float32))
     wh, wl = split_round(w_s)
     inv = np.float32(1.0 / (64.0 * 2.0 ** k2))
     main = np.stack([dot32(ah[:, None, :], wh[None, :, :])])[0]
@@ -72,3 +59,26 @@ def test_truncation_split_keeps_22_bits():
     rec = hi.astype(np.float64) + lo.astype(np.float64)
     err = np.abs(rec - s.astype(np.float64))
     assert np.all(err <= np.maximum(2.0 ** -22 * np.abs(s), 2.0 ** -25))
+
+
+@pytest.fixture(scope="module")
+def modelled_ratios():
+    """{path: (least, worst) ratio} of a contraction's max-abs error to that of torch's CPU float32 1x1 convolution, over
+    K = 64 .. 512 (the layers' Cin) and three seeds."""
+    worst = {}
+    for K in (64, 128, 256, 512):
+        for seed in range(3):
+            for path, r in error_ratios(K, seed).items():
+                worst.setdefault(path, []).append(r)
+    return {path: (min(rs), max(rs)) for path, rs in worst.items()}
+
+
+def test_launch_parity_multiples_follow_the_model(modelled_ratios):
+    """tests/test_launch_parity_gpu.py bounds each launch by MULT[path] x the unit's float32 error.  The multiples were set
+    at 2x the worst modelled ratio; 1.5x is required here because the float32 reference's reduction order depends on the
+    CPU.  The 3-pass bar stays far below what a single fp16 pass reaches."""
+    print({path: "%.2f .. %.2f" % r for path, r in modelled_ratios.items()})
+    for path in ("simt", "tc", "tc_fast"):
+        assert U.MULT[path] >= 1.5 * modelled_ratios[path][1], path
+    assert U.MULT["tc"] <= 3 * modelled_ratios["tc"][1]                 # ... and not much more
+    assert modelled_ratios["tc_fast"][0] > 50 * U.MULT["tc"]
